@@ -54,6 +54,29 @@ TUBE_L = (1.0, 0.0, 0.0, 0.0, 2.0, 1.0, 0.0, 0.0)               # namelist/tube_
 TUBE_R = (0.2, 1.186, 2.967, 0.0, 0.1368, 1.0, 1.6405, 0.0)
 MHD_BYTES_PER_CELL = 176.0   # 2 * 11 stored variables * 8 B (SURVEY 8d)
 BYTES_PER_CELL = 80.0   # algorithmic: read uold once + write unew once = 2*nvar*8 B (SURVEY 8d)
+# --dump-outputs: cells of the state sample per workload; the default line runs four workloads: (5+5+11+5) * 8 B * 2^17 = 27 MB
+DUMP_CELLS = 1 << 17
+DUMP_SEED = 20240611
+
+
+def dump_outputs(outdir, workload, uold, cells, dts):
+    """--dump-outputs: what the timed steps of `workload` hand back to the caller, after the last of them.
+    <workload>_state.npy: the conserved state uold[:, c] (float64, [nvar][n]) of a fixed, seeded sample of n <= DUMP_CELLS of the
+    active cells `cells` (all of them when fewer); <workload>_dt.npy: the time step of every timed step.  Same arguments, same
+    inputs and same sample, so two builds can be compared array for array."""
+    os.makedirs(outdir, exist_ok=True)
+    cells = np.asarray(cells, dtype=np.int64)
+    if len(cells) > DUMP_CELLS:
+        cells = cells[np.sort(np.random.default_rng(DUMP_SEED).choice(len(cells), DUMP_CELLS, replace=False))]
+    np.save(os.path.join(outdir, f"{workload}_state.npy"), np.ascontiguousarray(uold[:, cells], dtype=np.float64))
+    np.save(os.path.join(outdir, f"{workload}_dt.npy"), np.asarray(dts, dtype=np.float64))
+
+
+def active_cells(a, levels):
+    """0-based indices into the ncell axis of uold of the active cells of `levels` (oct order, then the 2^ndim cells)"""
+    T = 1 << a.ndim
+    return np.concatenate([(a.ncoarse + np.arange(T)[None, :] * a.ngridmax + a.active[l].astype(np.int64)[:, None] - 1).ravel()
+                           for l in levels])
 
 
 def sedov_ic(boxlen, nx, level):
@@ -173,12 +196,17 @@ def amr_bench(args, w, rank, world, local_rank, workload=None, embedded=False):
     l0 = launches0()
     h.synchronize(); torch.cuda.synchronize()
     t0 = time.perf_counter()
-    h.amr_steps(levelmin, nsub, steps)        # rgpu_amr_steps: time steps stay on the device, one host sync at the end
+    dts = h.amr_steps(levelmin, nsub, steps)  # rgpu_amr_steps: time steps stay on the device, one host sync at the end
     h.synchronize(); torch.cuda.synchronize()
     wall_host = time.perf_counter() - t0
     wall = h.level_info(levelmin).last_steps_ms * 1e-3      # CUDA events on the launching stream around the K coarse steps
     launches = launches0() - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        initial = a.uold.copy()           # the end-to-end pass below starts from the initial state, as without the dump
+        h.download_state(0)
+        dump_outputs(args.dump_outputs, workload or args.workload, a.uold, active_cells(a, range(levelmin, levelmax + 1)), dts)
+        a.uold[:] = initial
     # end to end: host arrays in, host arrays out around every coarse step
     t0 = time.perf_counter()
     for _ in range(args.e2e_steps):
@@ -526,6 +554,8 @@ def dense_bench(args, workload, rank, world, local_rank, secondary=False):
 
     # ---- correctness inside the bench: the state after warmup+steps level steps must be the single-GPU state, bit for bit
     h.download_state(level)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, workload, a.uold, active_cells(a, [level]), dts)
     check = None
     if not mhd:
         check = canonical_check(a, level, coarse, rank, np.concatenate([dts_w, dts]), keep_block=True)
@@ -699,7 +729,12 @@ def main():
     ap.add_argument("--order", default="lattice", choices=["lattice", "creation", "random"],
                     help="oct numbering of the fabricated tree; 'creation' = the reference's refine order (nvector = infinity)")
     ap.add_argument("--write-golden", action="store_true", help="single-GPU run: record the state / dt hashes in tests/golden/bench_hashes.json")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of each workload, write a fixed sample of the state they computed and their time "
+                         "steps as DIR/<workload>_{state,dt}.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

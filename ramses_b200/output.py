@@ -11,9 +11,9 @@ turns them into an `output_NNNNN/` directory that the reference's own tools read
     header_NNNNN.txt             amr/output_amr.f90:497-575  output_header (particle families, all zero)
 
 `read_snapshot` is the restart side (amr/init_amr.f90:227-520, hydro/init_hydro.f90:57-250).
-Serial runs (ncpu=1) and the Hilbert ordering header only.  tests/test_output_format.py reads the files back with the
-reference's reader and checker (tests/visu/visu_ramses.py: load_snapshot + check_solution) and so closes the loop
-state -> reference file format -> reference reader -> reference golden sums.
+Serial runs (ncpu=1) and the Hilbert ordering header only.  tests/test_output_format.py holds the files to the bytes the
+reference's reader and checker (tests/visu/visu_ramses.py: load_snapshot + check_solution) read, with what they returned
+stored under tests/golden/, and so closes the loop state -> reference file format -> reference reader -> reference golden sums.
 """
 import os
 import struct

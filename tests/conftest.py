@@ -27,8 +27,7 @@ IMPL = [dict(type="square", x_center=0.5, y_center=0.5, length_x=1.0, length_y=1
 IMPL_BOUND = [(1, (0, 0), (1, 1), (0, 0)), (2, (2, 2), (1, 1), (0, 0)), (4, (0, 2), (2, 2), (0, 0)), (3, (0, 2), (0, 0), (0, 0))]
 
 
-@pytest.fixture(scope="session")
-def implosion_run(orc):
+def make_implosion_run():
     from oracle.amr import FastAmrRun
     r = FastAmrRun(2, 5, 8, (1, 1, 1, 1, 0, 0), 1.0, nsubcycle=[2] * 10, nexpand=[4], ngridmax=100000, riemann="hllc",
                    slope_type=2, gamma=1.4, courant_factor=0.8, err_grad_d=0.05, err_grad_u=0.05, err_grad_p=0.05,
@@ -36,9 +35,18 @@ def implosion_run(orc):
     return r, r.run()
 
 
-@pytest.fixture(scope="session")
-def orszag_run(orc):
+def make_orszag_run():
     from oracle.amr_mhd import MhdAmrRun2D
     r = MhdAmrRun2D(5, 9, 1.0, nsubcycle=[1], riemann="hlld", riemann2d="hlld", slope_type=2, gamma=1.6666667,
                     courant_factor=0.8, err_grad_p=0.1, interpol_type=2, tout=[0.5], nexpand=1, ngridmax=100000)
     return r, r.run()
+
+
+@pytest.fixture(scope="session")
+def implosion_run(orc):
+    return make_implosion_run()
+
+
+@pytest.fixture(scope="session")
+def orszag_run(orc):
+    return make_orszag_run()

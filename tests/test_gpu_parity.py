@@ -435,3 +435,30 @@ def test_fast_mode_within_tolerance(gpu, riemann, ic):
     assert max_rel_err(uf, ref[:, idx]) <= 1e-12
     assert np.allclose(out[True][1], out[False][1], rtol=1e-12, atol=0)
     assert np.allclose(out[True][1], dts_ref, rtol=1e-12, atol=0)
+
+
+def test_bench_dump_outputs(gpu, tmp_path):
+    """bench.py --dump-outputs: after the --steps timed steps it writes their time steps and the seeded sample of the state they
+    computed, in float64; the run's own check finds that state equal to the recorded single-GPU hashes (bench_hashes.json), and a
+    second run with the same arguments writes the same arrays bit for bit."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--workload", "sedov3d_128_hllc", "--steps", "5", "--warmup", "3",
+               "--no-cpu-baseline", "--no-fast", "--e2e-steps", "1", "--dump-outputs", str(d)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 5 and line["check"]["equals_single_gpu_golden"] is True
+        assert sorted(os.listdir(d)) == ["sedov3d_128_hllc_dt.npy", "sedov3d_128_hllc_state.npy"]
+        out.append({f: np.load(d / f) for f in os.listdir(d)})
+    dt, state = out[0]["sedov3d_128_hllc_dt.npy"], out[0]["sedov3d_128_hllc_state.npy"]
+    assert dt.dtype == np.float64 and dt.shape == (5,) and (dt > 0).all()
+    assert state.dtype == np.float64 and state.shape == (5, 1 << 17) and np.isfinite(state).all()
+    for f in out[0]:
+        assert np.array_equal(out[0][f], out[1][f]), f

@@ -1,18 +1,21 @@
-"""ramses_b200/output.py writes the reference's snapshot format; the files are read back with the REFERENCE's own reader and
-checked with the REFERENCE's own check_solution (tests/visu/visu_ramses.py) against the golden sums: state -> reference file
-format -> reference reader -> reference checker.  Needs the reference tree (only present in the build container): skipped on
-machines without it."""
+"""ramses_b200/output.py writes the reference's snapshot format: state -> reference file format -> reference reader -> reference
+checker.  The reference's own reader and checker (tests/visu/visu_ramses.py of the reference: load_snapshot + check_solution)
+were run on the snapshots these tests write by tests/golden/make_snapshot_golden.py, and what they returned is stored:
+
+  golden/snapshot_golden.json  per snapshot: the SHA-256 of every file of output_NNNNN/ the reader was given; for the two long
+                               runs also the sums check_solution computed and its verdict against the reference's golden file
+  golden/snapshot_<name>.npz   the per-cell arrays and scalars load_snapshot returned (short runs)
+
+Each test writes its snapshot again and requires the same bytes, so the reference reader would return the stored arrays; those
+arrays are then compared with the run as the reader's live output was."""
+import hashlib
 import json
 import os
-import sys
 
 import numpy as np
-import pytest
 
-REF_VISU = "/root/reference/tests/visu"
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF_VISU, "visu_ramses.py")),
-                                reason="reference tree not available")
+SNAPSHOT_GOLDEN = os.path.join(GOLD, "snapshot_golden.json")
 
 
 def _write_from_run(r, tmp, iout, mhd=False):
@@ -32,95 +35,25 @@ def _write_from_run(r, tmp, iout, mhd=False):
         dtnew=[r.dtnew[l] for l in range(1, L + 1)], nstep=r.nstep, nstep_coarse=r.nstep_coarse, tout=r.tout, mhd=mhd)
 
 
-def _check_with_reference(tmp, iout, test_name, ref_json):
-    sys.path.insert(0, REF_VISU)
-    try:
-        import visu_ramses
-    finally:
-        sys.path.remove(REF_VISU)
-    ref = json.load(open(os.path.join(GOLD, ref_json)))
-    cwd = os.getcwd()
-    os.chdir(str(tmp))
-    try:
-        with open(test_name + "-ref.dat", "w") as f:
-            for k in sorted(ref):
-                f.write("%s : %.16e\n" % (k, ref[k]))
-        data = visu_ramses.load_snapshot(iout)
-        visu_ramses.check_solution(data["data"], test_name)       # what tests/*/plot-*.py end with; prints PASSED
-    finally:
-        os.chdir(cwd)
-    return data
-
-
-def test_sod_tube_snapshot_through_reference_reader(orc, tmp_path, capsys):
+# ---- the snapshots (also run by tests/golden/make_snapshot_golden.py) ------------------------------------------------------
+def sod_run():
     from oracle.amr import AmrRun
     from test_oracle_golden import SOD
     r = AmrRun(1, 3, 10, (1, 1, 0, 0, 0, 0), 1.0, nsubcycle=[1, 1, 1, 2], nexpand=1, ngridmax=2000, riemann="hllc",
                slope_type=2, gamma=1.4, courant_factor=0.8, err_grad_d=0.05, err_grad_u=0.05, err_grad_p=0.05,
                interpol_type=2, interpol_var=0, regions=SOD, tout=[0.245])
-    snap = r.run()
-    # the driver stops after the output step: the state at the output time is the current one
-    _write_from_run(r, tmp_path, 2)
-    data = _check_with_reference(tmp_path, 2, "sod-tube", "sod_tube_ref.json")
-    assert "PASSED" in capsys.readouterr().out              # the reference's own verdict on the reference's own golden file
-    assert data["data"]["ncells"] == 142 and abs(data["data"]["time"] - snap["t"]) < 1e-14
-    rows = snap["rows"]
-    x = np.array([q[1][0] for q in rows])
-    order_ref, order_ours = np.argsort(data["data"]["x"]), np.argsort(x)
-    assert np.array_equal(np.sort(data["data"]["x"]), np.sort(x))
-    assert np.array_equal(data["data"]["density"][order_ref], np.array([q[2] for q in rows])[order_ours])
-    assert np.array_equal(data["data"]["pressure"][order_ref], np.array([q[4] for q in rows])[order_ours])
+    return r, r.run()
 
 
-def test_orszag_tang_snapshot_through_reference_reader(orc, tmp_path):
-    """a short NDIM=2 MHD AMR run: the eleven output fields survive the file format bit for bit"""
+def orszag_short_run():
     from oracle.amr_mhd import MhdAmrRun2D
     r = MhdAmrRun2D(4, 6, 1.0, nsubcycle=[1], riemann="hlld", riemann2d="hlld", slope_type=2, gamma=1.6666667, courant_factor=0.8,
                     err_grad_p=0.1, interpol_type=2, tout=[0.1], nexpand=1, ngridmax=20000)
-    snap = r.run()
-    _write_from_run(r, tmp_path, 2, mhd=True)
-    sys.path.insert(0, REF_VISU)
-    try:
-        import visu_ramses
-    finally:
-        sys.path.remove(REF_VISU)
-    cwd = os.getcwd()
-    os.chdir(str(tmp_path))
-    try:
-        data = visu_ramses.load_snapshot(2)
-    finally:
-        os.chdir(cwd)
-    ours = snap["rows"]
-    assert data["data"]["ncells"] == len(ours["level"])
-    key_ref = np.lexsort((data["data"]["y"], data["data"]["x"]))
-    key_our = np.lexsort((ours["y"], ours["x"]))
-    for k in ("level", "x", "y", "dx", "density", "velocity_x", "velocity_y", "velocity_z", "pressure", "B_x_left", "B_y_left",
-              "B_z_left", "B_x_right", "B_y_right", "B_z_right"):
-        assert np.array_equal(np.asarray(data["data"][k])[key_ref], np.asarray(ours[k])[key_our]), k
+    return r, r.run()
 
 
-def test_implosion_and_orszag_tang_through_reference_checker(implosion_run, orszag_run, tmp_path, capsys):
-    """the two long golden runs (session fixtures shared with test_oracle_golden.py): write the final state in the reference's
-    format and let the REFERENCE's check_solution compare with the REFERENCE's golden file -- it prints PASSED for orszag-tang
-    (all sums to 2e-15) and for implosion (within its 3e-13 tolerance)."""
-    r, _ = orszag_run
-    d1 = tmp_path / "ot"
-    d1.mkdir()
-    _write_from_run(r, d1, 2, mhd=True)
-    _check_with_reference(d1, 2, "orszag-tang", "orszag_tang_ref.json")
-    assert "PASSED" in capsys.readouterr().out
-    r, _ = implosion_run
-    d2 = tmp_path / "impl"
-    d2.mkdir()
-    _write_from_run(r, d2, 2)
-    _check_with_reference(d2, 2, "implosion", "implosion_ref.json")
-    assert "PASSED" in capsys.readouterr().out
-
-
-def test_snapshot_from_host_mirror_nested_tree(tmp_path):
-    """the product's host mirror (AmrCommons from ramses_b200.tree.build_nested_tree, three levels) -> snapshot -> reference
-    reader: every leaf cell comes back at its position with its value."""
-    from ramses_b200.output import snapshot_from_commons
+def host_mirror_commons():
+    """the product's host mirror (AmrCommons from ramses_b200.tree.build_nested_tree, three levels) with a linear state"""
     from ramses_b200.tree import build_nested_tree, fill_state
     a = build_nested_tree(3, 5, half_width=2)
     a.gamma = 1.4
@@ -133,18 +66,99 @@ def test_snapshot_from_host_mirror_nested_tree(tmp_path):
         return u
     for l in range(1, 6):
         fill_state(a, l, fn)
-    snapshot_from_commons(a, str(tmp_path), 1, t=0.125, levelmin=3)
-    sys.path.insert(0, REF_VISU)
-    try:
-        import visu_ramses
-    finally:
-        sys.path.remove(REF_VISU)
-    cwd = os.getcwd()
-    os.chdir(str(tmp_path))
-    try:
-        data = visu_ramses.load_snapshot(1)["data"]
-    finally:
-        os.chdir(cwd)
+    return a
+
+
+def write_host_mirror(a, outdir):
+    from ramses_b200.output import snapshot_from_commons
+    return snapshot_from_commons(a, str(outdir), 1, t=0.125, levelmin=3)
+
+
+def file_hashes(snapdir):
+    """SHA-256 of every file of an output_NNNNN/ directory"""
+    return {f: hashlib.sha256(open(os.path.join(snapdir, f), "rb").read()).hexdigest() for f in sorted(os.listdir(snapdir))}
+
+
+# ---- what the reference's reader and checker returned ----------------------------------------------------------------------
+def _golden(name):
+    return json.load(open(SNAPSHOT_GOLDEN))[name]
+
+
+def _assert_reader_input(snapdir, name):
+    """the snapshot holds the bytes the reference reader was given when the golden arrays were recorded"""
+    assert file_hashes(snapdir) == _golden(name)["files"], f"{name}: the snapshot files differ from those the reference reader read"
+
+
+def _reader_output(name):
+    z = np.load(os.path.join(GOLD, "snapshot_%s.npz" % name))
+    return {k: z[k] for k in z.files}
+
+
+def _assert_checker_passed(name, ref_json):
+    """check_solution's sums of the reference reader's data against the reference's golden file: its verdict, and its comparison
+    (relative difference <= 3e-13 per variable, tests/visu/visu_ramses.py:497 of the reference) redone on the stored sums"""
+    g = _golden(name)
+    assert g["check_solution"] == "PASSED"
+    ref = json.load(open(os.path.join(GOLD, ref_json)))
+    sums = g["sums"]
+    assert sorted(sums) == sorted(ref)
+    for k, v in ref.items():
+        s = sums[k]
+        err = 0.0 if s == v == 0.0 else abs(s - v) / min(abs(s), abs(v))
+        assert err <= 3.0e-13, (name, k, s, v, err)
+
+
+def test_sod_tube_snapshot_through_reference_reader(orc, tmp_path):
+    r, snap = sod_run()
+    # the driver stops after the output step: the state at the output time is the current one
+    _assert_reader_input(_write_from_run(r, tmp_path, 2), "sod_tube")
+    _assert_checker_passed("sod_tube", "sod_tube_ref.json")   # the reference's own verdict on the reference's own golden file
+    data = _reader_output("sod_tube")
+    assert data["ncells"] == 142 and abs(data["time"] - snap["t"]) < 1e-14
+    rows = snap["rows"]
+    x = np.array([q[1][0] for q in rows])
+    order_ref, order_ours = np.argsort(data["x"]), np.argsort(x)
+    assert np.array_equal(np.sort(data["x"]), np.sort(x))
+    assert np.array_equal(data["density"][order_ref], np.array([q[2] for q in rows])[order_ours])
+    assert np.array_equal(data["pressure"][order_ref], np.array([q[4] for q in rows])[order_ours])
+
+
+def test_orszag_tang_snapshot_through_reference_reader(orc, tmp_path):
+    """a short NDIM=2 MHD AMR run: the eleven output fields survive the file format bit for bit"""
+    r, snap = orszag_short_run()
+    _assert_reader_input(_write_from_run(r, tmp_path, 2, mhd=True), "orszag_tang_short")
+    data = _reader_output("orszag_tang_short")
+    ours = snap["rows"]
+    assert data["ncells"] == len(ours["level"])
+    key_ref = np.lexsort((data["y"], data["x"]))
+    key_our = np.lexsort((ours["y"], ours["x"]))
+    for k in ("level", "x", "y", "dx", "density", "velocity_x", "velocity_y", "velocity_z", "pressure", "B_x_left", "B_y_left",
+              "B_z_left", "B_x_right", "B_y_right", "B_z_right"):
+        assert np.array_equal(np.asarray(data[k])[key_ref], np.asarray(ours[k])[key_our]), k
+
+
+def test_implosion_and_orszag_tang_through_reference_checker(implosion_run, orszag_run, tmp_path):
+    """the two long golden runs (session fixtures shared with test_oracle_golden.py): the final state in the reference's format
+    is what the REFERENCE's check_solution compared with the REFERENCE's golden file -- PASSED for orszag-tang (all sums to
+    2e-15) and for implosion (within its 3e-13 tolerance)."""
+    r, _ = orszag_run
+    d1 = tmp_path / "ot"
+    d1.mkdir()
+    _assert_reader_input(_write_from_run(r, d1, 2, mhd=True), "orszag_tang")
+    _assert_checker_passed("orszag_tang", "orszag_tang_ref.json")
+    r, _ = implosion_run
+    d2 = tmp_path / "impl"
+    d2.mkdir()
+    _assert_reader_input(_write_from_run(r, d2, 2), "implosion")
+    _assert_checker_passed("implosion", "implosion_ref.json")
+
+
+def test_snapshot_from_host_mirror_nested_tree(tmp_path):
+    """the product's host mirror (AmrCommons from ramses_b200.tree.build_nested_tree, three levels) -> snapshot -> reference
+    reader: every leaf cell comes back at its position with its value."""
+    a = host_mirror_commons()
+    _assert_reader_input(write_host_mirror(a, tmp_path), "host_mirror")
+    data = _reader_output("host_mirror")
     nleaf = sum(int((a.son[a.ncoarse + ind * a.ngridmax + a.active[l].astype(np.int64) - 1] == 0).sum())
                 for l in range(1, 6) for ind in range(8))
     assert data["ncells"] == nleaf and data["time"] == 0.125
